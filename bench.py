@@ -311,6 +311,45 @@ def placement_parity(topo, specs, sample, gblob, result, oracle_threads):
     return bad
 
 
+# ------------------------------------------------------------------ outputs
+DUMP_LIMIT = 64_000_000   # bytes --dump-outputs writes at most, .npy headers included
+
+
+def _seeded_sample(n, k, seed):
+    """Sorted indices of a fixed sample of k of range(n); all of them when k >= n."""
+    if k >= n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+
+
+def dump_outputs(path, placement, read_row=None, n_rows=0, n_cols=0, col0=0):
+    """Writes what a caller of the timed path received from its last step, one DIR/<name>.npy per array, so that two
+    builds run with the same arguments (hence the same seeded inputs) can be compared output for output:
+    assign / status / domain as float64 (exact for int32) and, when the path keeps one, the dense score matrix as
+    float32 (bit for bit).  An infeasible (replica, node) pair scores -inf (DESIGN.md §3.3); every file holds finite
+    values, so such entries are written as 0 in scores and as 0 in scores_feasible (1 elsewhere).  The matrix is far
+    larger than DUMP_LIMIT at the default sizes, so it is written as a fixed sample: rows, and columns when one row
+    alone would not fit, drawn by seeded generators; scores_rows / scores_cols hold the row and node indices of the
+    sample.  read_row(r) returns row r over nodes [col0, col0 + n_cols)."""
+    os.makedirs(path, exist_ok=True)
+    out = {name: np.asarray(a, dtype=np.float64) for name, a in zip(("assign", "status", "domain"), placement)}
+    budget = DUMP_LIMIT - 7 * 4096 - sum(a.nbytes for a in out.values())   # seven files, a header of < 4 KB each
+    if budget < 0:
+        raise SystemExit(f"--dump-outputs: the placement alone is larger than {DUMP_LIMIT} bytes")
+    if read_row is not None and n_rows > 0:
+        cols = _seeded_sample(n_cols, budget // 32, seed=1)   # 8 B of index + >= 2 rows of 8 B (score, feasible) per column
+        rows = _seeded_sample(n_rows, (budget - 8 * len(cols)) // (8 * len(cols) + 8), seed=2)
+        scores = np.stack([read_row(int(r))[cols] for r in rows]).astype(np.float32, copy=False)
+        feasible = scores != -np.inf
+        out["scores"] = np.where(feasible, scores, np.float32(0))
+        out["scores_feasible"] = feasible.astype(np.float32)
+        out["scores_rows"] = rows.astype(np.float64)
+        out["scores_cols"] = (col0 + cols).astype(np.float64)
+    assert sum(a.nbytes for a in out.values()) <= DUMP_LIMIT
+    for name, a in out.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 # ------------------------------------------------------------------- ours
 class Dist:
     def __init__(self, args):
@@ -389,9 +428,10 @@ def make_device_step(D, eng, handles, n_waves, mode):
     return step
 
 
-def run_config(D, args, cfg_name, with_clocks):
+def run_config(D, args, cfg_name, with_clocks, dump_dir=None):
     """Stages one configuration, checks it against the oracle, times the resident-plan leg
-    (`value`) and the host-buffer leg (`e2e`).  Returns the pieces of the JSON line."""
+    (`value`) and the host-buffer leg (`e2e`).  Returns the pieces of the JSON line.
+    dump_dir: rank 0 writes there what the last step of the leg `value` times computed (dump_outputs)."""
     torch = D.torch
     from rbg_b200 import synth
     from rbg_b200.engine import TopoPlacer
@@ -490,6 +530,9 @@ def run_config(D, args, cfg_name, with_clocks):
         dev_ms = ev0.elapsed_time(ev1)
         launches = eng.stats()["kernel_launches"] - launches0
         post = [eng.fetch(h) for h in handles]
+        if dump_dir and rank == 0:   # step k of the timed region placed batch handles[k % slots]
+            last = (steps - 1) % slots
+            dump_outputs(dump_dir, post[last], lambda r: eng.read_scores(handles[last], r), total_r, hi - lo, lo)
         if slots > 1:   # every slot holds the same fleet: the chained passes must leave what the checked pass left
             rows = sorted(set(int(i) for i in np.linspace(0, total_r - 1, 16)))
             ref_rows = [eng.read_scores(handles[0], r).copy() for r in rows]
@@ -631,6 +674,8 @@ def run_config(D, args, cfg_name, with_clocks):
         torch.cuda.synchronize()
         rounds.append((time.perf_counter() - t0) * 1e3)
     e2e_ms = D.max_over_ranks(sorted(rounds)[len(rounds) // 2])
+    if churn and dump_dir and rank == 0:   # the host-buffer call is the timed path here; it keeps no matrix
+        dump_outputs(dump_dir, res)
     if not churn:
         # the host-buffer entry point (direct path) against the staged plan the oracle checked above: assignment, status, domain
         assert all(np.array_equal(x, y) for x, y in zip(fetched, res)), "e2e placement differs from the staged path"
@@ -686,7 +731,7 @@ def roofline_of(r, peak, peak_src):
 def run_ours(args):
     D = Dist(args)
     rank, world = D.rank, D.world
-    main = run_config(D, args, args.config, with_clocks=True)
+    main = run_config(D, args, args.config, with_clocks=True, dump_dir=args.dump_outputs)
     alts = {}
     if args.alt:
         for name in ("cfg4", "cfg5"):
@@ -858,7 +903,12 @@ def main():
                     help="staged copies of the fleet re-placed round robin in the resident leg (independent batches, one per "
                          "step); > 1 chains the dense-matrix kernel of a step behind the selection kernel of the step before it")
     ap.add_argument("--soak", type=float, default=0.6, help="seconds of untimed identical steps before the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64, "
+                         "at most 64 MB: a fixed seeded sample of the score matrix), rank 0 only")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the GPU path computed: it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:
